@@ -19,6 +19,10 @@ N > 1 (torchrun): node-sharded run (SURVEY.md §8e), weak scaling: the cluster g
 a contiguous block of the node axis, the per-wave exchange of shard winners happens inside the persistent kernel over peer
 memory (NVLink), torch.distributed (NCCL) only carries the IPC handles and the final small reductions. value = evals of the
 whole job / max-over-ranks time. `--mode replicas` runs N independent single-GPU analyses instead (no data-path collective).
+
+--dump-outputs DIR: after the timed steps, the result of the last timed step (what a caller of ccsim_run receives: pod -> node
+sequence, FitError histogram, placed count, stop code, preemption counts) is written as DIR/<name>.npy in float64. The
+workloads are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import importlib
@@ -31,6 +35,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark leaves the tree as the build left it (it may be read-only)
 
 import numpy as np  # noqa: E402
 
@@ -182,6 +187,25 @@ def parity_block(got, want, pods):
             "against": "oracle/ccsim_oracle.c (canonical mode), same snapshot", "first_mismatch": first_bad}
 
 
+DUMP_MAX_POD_NODE = 3 << 20    # float64 values + positions of a sampled pod -> node sequence stay under 64 MB in all
+
+
+def dump_outputs(out_dir, r):
+    """Writes a run result (dict: placed, stop_code, pod_node, reason_hist, preempt_no_victims, preempt_not_helpful) as
+    <out_dir>/<name>.npy in float64 (exact for these integer outputs). A pod -> node sequence longer than DUMP_MAX_POD_NODE is
+    replaced by a fixed seeded sample of its positions, written alongside as pod_node_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = {k: np.asarray(r[k], np.float64) for k in ("placed", "stop_code", "reason_hist", "preempt_no_victims", "preempt_not_helpful")}
+    pod_node = np.asarray(r["pod_node"], np.float64)
+    if len(pod_node) > DUMP_MAX_POD_NODE:
+        idx = np.sort(np.random.default_rng(0).choice(len(pod_node), DUMP_MAX_POD_NODE, replace=False))
+        pod_node = pod_node[idx]
+        out["pod_node_index"] = idx.astype(np.float64)
+    out["pod_node"] = pod_node
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def objects_leg(flat, device, steps):
     """e2e through the reference-facing API (include/cchost.h = pkg/framework's New / SyncWithClient / Run / Report): the C4
     cluster as v1.Node / v1.Pod JSON in host memory (what SyncWithClient LISTs, simulator.go:176-295) -> C++ ingest + NodeInfo
@@ -265,7 +289,7 @@ def run_reference(args):
     if rank != 0:
         return
     snap, tmpl, ctr = MAKE(world if args.mode == "sharded" else 1)     # the same workload as our arm at this N
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     evals = placed = 0
     dt = 0.0
     threads = cores = pods = 0
@@ -275,6 +299,8 @@ def run_reference(args):
         evals += r.evals
         placed += r.placed
         dt += d
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, vars(r))
     val = evals / dt
     line = {
         "impl": "reference", "metric": "predicate-evals/sec", "value": val, "unit": "evals/s", "n_gpus": args.gpus,
@@ -332,7 +358,10 @@ def main():
     ap.add_argument("--no-objects", action="store_true", help="skip the e2e_objects leg (plugin call from Node/Pod JSON)")
     ap.add_argument("--workload", default="c4", choices=sorted(WORKLOADS), help="c4 (default: the metric's 100k-node configuration) or c5 (1M nodes x 64 podspecs)")
     ap.add_argument("--mode", default="sharded", choices=["sharded", "replicas"], help="N>1: node-sharded run or independent replicas")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's result as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     select_workload(args.workload)
     if args.impl == "reference":
         return run_reference(args)
@@ -398,7 +427,7 @@ def main():
         last_result = sharded.merge_results(dist, res)
     else:
         last_result = {"placed": res.placed, "stop_code": res.stop_code, "pod_node": res.pod_node, "reason_hist": res.reason_hist,
-                       "preempt_no_victims": res.preempt_no_victims}
+                       "preempt_no_victims": res.preempt_no_victims, "preempt_not_helpful": res.preempt_not_helpful}
     flushes = args.steps
     launches = eng.kernel_launches() - launches0 - flushes
     t_total = sum(step_wall)
@@ -494,8 +523,10 @@ def main():
             line["parity"] = None
         # ---- the reference-facing plugin call: framework.New + SyncWithClient + Run + Report from Node / Pod JSON in host memory ----
         if WKEY == "c4" and world == 1 and not args.no_objects:
-            line["e2e_objects"] = objects_leg(last_result, local, max(1, min(args.steps, 2)))
+            line["e2e_objects"] = objects_leg(last_result, local, args.steps)
             parity_ok = parity_ok and line["e2e_objects"]["same_sequence_as_flat_run"]
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_result)
         print(json.dumps(line), flush=True)
     eng.close()
     if world > 1:
