@@ -70,6 +70,12 @@ REASON_TEXT = {
 STOP_UNSCHEDULABLE, STOP_LIMIT_REACHED = 0, 1
 ENGINE_AUTO, ENGINE_SEQUENTIAL, ENGINE_BATCHED = 0, 1, 2
 SAMPLING_CANONICAL, SAMPLING_REFERENCE = 0, 1
+# ccsim_run_stats out[0]: engine code in the low byte, the wave kernel's instantiation above it
+KV_ENGINE_MASK = 0xFF
+KV_RESIDENT = 1 << 8
+KV_STREAM_MODE_SHIFT = 9
+KV_REFERENCE_SAMPLING = 1 << 11
+KV_CROSS_GPU = 1 << 12
 
 P64 = C.POINTER(C.c_int64)
 P32 = C.POINTER(C.c_int32)

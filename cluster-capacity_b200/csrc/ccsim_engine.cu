@@ -710,6 +710,19 @@ __global__ void ccsim_count_kernel(const int32_t *pod_node, long long placed, in
   }
 }
 
+// ccsim_debug_node_scores: score_node (and its two parts) of every node, `clones` pods of the template after the snapshot
+__global__ void ccsim_debug_score_kernel(int32_t n, const int64_t *a_cpu, const int64_t *a_mem, const int64_t *r_cpu, const int64_t *r_mem,
+                                         const int64_t *z_cpu, const int64_t *z_mem, const ccsim_template t, ScoreWeights sw, int64_t clones,
+                                         int64_t *total, int64_t *least, int64_t *balanced) {
+  for (int32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const int64_t lq_cpu = z_cpu[i] + clones * t.nz_cpu + t.least_cpu, lq_mem = z_mem[i] + clones * t.nz_mem + t.least_mem;
+    const int64_t bq_cpu = r_cpu[i] + clones * t.req_cpu + t.bal_cpu, bq_mem = r_mem[i] + clones * t.req_mem + t.bal_mem;
+    total[i] = score_node(a_cpu[i], a_mem[i], lq_cpu, lq_mem, bq_cpu, bq_mem, sw);
+    least[i] = score_least(a_cpu[i], a_mem[i], lq_cpu, lq_mem, sw.least_w_cpu, sw.least_w_mem);
+    balanced[i] = score_balanced(a_cpu[i], a_mem[i], bq_cpu, bq_mem);
+  }
+}
+
 __global__ void ccsim_flush_kernel(unsigned long long *buf, size_t n, unsigned long long v) {
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) buf[i] = v + i;
 }
@@ -723,6 +736,7 @@ struct RunPlan {      // what run_prepare decided, consumed by the launch
   DevParams p; LeanParams lp; MultiParams mp; StreamParams sp;
   const void *kern = nullptr; int grid = 0, block = 0; size_t smem = 0;
   bool stream = false, multi = false, batched = false, lean = false, resident = false;
+  int64_t variant = 0;   // CCSIM_KV_* bits of the instantiation (ccsim_run_stats out[0] above the engine code)
 };
 
 struct ccsim_handle {
@@ -1405,6 +1419,8 @@ static int run_prepare(ccsim_handle *h, int64_t max_pods) {
   if (occ < 1 || occ * h->sm_count < grid) return fail(h, CCSIM_ECUDA, "persistent grid %d does not fit (occupancy %d x %d SMs)", grid, occ, h->sm_count);
   pl.p = p; pl.lp = lp; pl.mp = mp; pl.sp = sp; pl.kern = kern; pl.grid = grid; pl.block = block; pl.smem = smem;
   pl.stream = stream; pl.multi = multi; pl.batched = batched; pl.lean = lean; pl.resident = resident;
+  pl.variant = (!stream && !lean && resident ? CCSIM_KV_RESIDENT : 0) | (stream ? (int64_t)stream_mode << CCSIM_KV_STREAM_MODE_SHIFT : 0) |
+               (lean && faithful ? CCSIM_KV_REFERENCE_SAMPLING : 0) | (multi && h->cfg.world > 1 ? CCSIM_KV_CROSS_GPU : 0);
   pl.valid = true;
   return CCSIM_OK;
 }
@@ -1465,10 +1481,10 @@ extern "C" int ccsim_run(ccsim_handle *h, int64_t max_pods, ccsim_result *out) {
   fprintf(stderr, "[ccsim phases 6/7] %.0f %.0f\n", (double)ho.phase_cycles[6] / ho.waves, (double)ho.phase_cycles[7] / ho.waves);
 #endif
   if (h->cfg.world > 1) h->xwave0 += (uint32_t)ho.waves;    // identical on every rank: the engines run the same waves everywhere
-  h->last_stat[0] = stream ? 4 : multi ? 3 : batched ? 2 : lean ? 1 : 0; h->last_stat[1] = ho.waves; h->last_stat[2] = ho.placed;
-  h->last_stat[3] = ho.stat[0]; h->last_stat[4] = ho.stat[1]; h->last_stat[5] = grid; h->last_stat[6] = block; h->last_stat[7] = (int64_t)smem;
+  h->last_stat[0] = (stream ? 4 : multi ? 3 : batched ? 2 : lean ? 1 : 0) | pl.variant; h->last_stat[1] = ho.waves; h->last_stat[2] = ho.placed;
+  h->last_stat[3] = ho.stat[0]; h->last_stat[4] = ho.stat[1]; h->last_stat[5] = grid; h->last_stat[6] = block;
+  h->last_stat[7] = ho.stat[2];   // multi-commit replay rounds
   for (int q = 0; q < 8; q++) h->last_stat[8 + q] = ho.phase_cycles[q];
-  h->last_stat[7] = ho.stat[2];   // (replay rounds; the shared-memory size is not needed by anybody)
   out->placed = ho.placed; out->stop_code = ho.stop_code; out->waves = ho.waves; out->evals = ho.evals; out->run_ms = ms;
   out->examined = ho.examined ? ho.examined : ho.evals;
   h->last_placed = ho.placed;
@@ -1526,6 +1542,33 @@ extern "C" int64_t ccsim_kernel_launches(const ccsim_handle *h) { return h ? h->
 extern "C" int ccsim_run_stats(const ccsim_handle *h, int64_t out[16]) {
   if (!h || !out) return CCSIM_EINVAL;
   memcpy(out, h->last_stat, sizeof(h->last_stat));
+  return CCSIM_OK;
+}
+
+extern "C" int ccsim_debug_node_scores(ccsim_handle *h, int32_t t, int32_t clones, int64_t *total, int64_t *least, int64_t *balanced) {
+  if (!h || !total || !least || !balanced) return fail(h, CCSIM_EINVAL, "null argument");
+  if (!h->have_templates || t < 0 || t >= h->n_templates) return fail(h, CCSIM_EINVAL, "template index");
+  if (clones < 0) return fail(h, CCSIM_EINVAL, "clones < 0");
+  CK(cudaSetDevice(h->cfg.device));
+  const int32_t n = h->n;
+  if (n == 0) return CCSIM_OK;
+  const ccsim_template &T = h->h_templates[t];
+  ScoreWeights sw;      // as the wave kernels fold it (lean_build_consts)
+  sw.w_fit = (T.score_enable & CCSIM_PL_FIT) ? T.w_fit : 0;
+  sw.w_balanced = ((T.score_enable & CCSIM_PL_BALANCED) && !(T.flags & CCSIM_TF_BALANCED_SKIP)) ? T.w_balanced : 0;
+  sw.least_w_cpu = T.least_w_cpu; sw.least_w_mem = T.least_w_mem;
+  int64_t *d = nullptr;
+  CK(cudaMalloc((void **)&d, (size_t)n * 3 * sizeof(int64_t)));
+  ccsim_debug_score_kernel<<<std::min(4 * h->sm_count, (n + 255) / 256), 256, 0, h->stream>>>(
+      n, h->d_alloc_cpu, h->d_alloc_mem, h->s_req_cpu, h->s_req_mem, h->s_nz_cpu, h->s_nz_mem, T, sw, clones, d, d + n, d + 2 * (size_t)n);
+  h->launches++;
+  cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess) e = cudaMemcpyAsync(total, d, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(least, d + n, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(balanced, d + 2 * (size_t)n, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+  cudaFree(d);
+  if (e != cudaSuccess) return fail(h, CCSIM_ECUDA, "ccsim_debug_node_scores: %s", cudaGetErrorString(e));
   return CCSIM_OK;
 }
 

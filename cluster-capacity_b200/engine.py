@@ -16,7 +16,8 @@ _lib = None
 
 EXPORTS = ["ccsim_create", "ccsim_destroy", "ccsim_last_error", "ccsim_abi_version", "ccsim_load_nodes",
            "ccsim_set_templates", "ccsim_run", "ccsim_prepare", "ccsim_node_counts", "ccsim_peer_export", "ccsim_peer_import",
-           "ccsim_device_info", "ccsim_kernel_launches", "ccsim_flush_l2", "ccsim_run_stats", "ccsim_peer_local", "ccsim_peer_import_local"]
+           "ccsim_device_info", "ccsim_kernel_launches", "ccsim_flush_l2", "ccsim_run_stats", "ccsim_peer_local", "ccsim_peer_import_local",
+           "ccsim_debug_node_scores"]
 
 
 class EngineError(RuntimeError):
@@ -58,6 +59,8 @@ def lib():
         L.ccsim_peer_import_local.argtypes = [C.c_void_p, C.c_int32, C.POINTER(C.c_void_p)]
         L.ccsim_run_stats.restype = C.c_int
         L.ccsim_run_stats.argtypes = [C.c_void_p, abi.P64]
+        L.ccsim_debug_node_scores.restype = C.c_int
+        L.ccsim_debug_node_scores.argtypes = [C.c_void_p, C.c_int32, C.c_int32, abi.P64, abi.P64, abi.P64]
         L.ccsim_peer_export.restype = C.c_int
         L.ccsim_peer_export.argtypes = [C.c_void_p, abi.PU8]
         L.ccsim_peer_import.restype = C.c_int
@@ -161,12 +164,39 @@ class Engine:
 
     ENGINE_NAMES = ("generic", "lean sequential", "tie-run batching", "multi-commit", "streaming (TMA)")
 
+    @staticmethod
+    def kernel_name(code):
+        """The wave kernel instantiation behind ccsim_run_stats out[0]: generic/resident, generic/streamed, lean/canonical,
+        lean/reference, batched, multi/1gpu, multi/shards, stream/mode0, stream/mode1 or stream/mode2."""
+        engine = code & abi.KV_ENGINE_MASK
+        if engine == 0:
+            return "generic/resident" if code & abi.KV_RESIDENT else "generic/streamed"
+        if engine == 1:
+            return "lean/reference" if code & abi.KV_REFERENCE_SAMPLING else "lean/canonical"
+        if engine == 2:
+            return "batched"
+        if engine == 3:
+            return "multi/shards" if code & abi.KV_CROSS_GPU else "multi/1gpu"
+        return "stream/mode%d" % ((code >> abi.KV_STREAM_MODE_SHIFT) & 3)
+
     def run_stats(self):
-        """Latency anatomy of the last run (see ccsim_run_stats in include/ccsim.h)."""
+        """Latency anatomy of the last run (see ccsim_run_stats in include/ccsim.h). "replay_rounds" was called "smem_bytes" (the
+        slot once held the shared-memory size); the old key stays for existing readers."""
         v = np.zeros(16, np.int64)
         self._check(lib().ccsim_run_stats(self._h, v.ctypes.data_as(abi.P64)), "ccsim_run_stats")
-        return {"engine": self.ENGINE_NAMES[int(v[0])], "waves": int(v[1]), "placed": int(v[2]), "candidates": int(v[3]), "bar_raised_waves": int(v[4]),
-                "grid": int(v[5]), "block": int(v[6]), "smem_bytes": int(v[7]), "phase_cycles": [int(x) for x in v[8:16]]}
+        code = int(v[0])
+        return {"engine": self.ENGINE_NAMES[code & abi.KV_ENGINE_MASK], "kernel": self.kernel_name(code), "waves": int(v[1]), "placed": int(v[2]),
+                "candidates": int(v[3]), "bar_raised_waves": int(v[4]), "grid": int(v[5]), "block": int(v[6]),
+                "replay_rounds": int(v[7]), "smem_bytes": int(v[7]), "phase_cycles": [int(x) for x in v[8:16]]}
+
+    def debug_node_scores(self, t, clones=0):
+        """Device scores of every node for template t after `clones` commits of it (see ccsim_debug_node_scores):
+        (total, least, balanced) int64 arrays of this handle's nodes."""
+        n = max(1, self._n)
+        total, least, balanced = np.zeros(n, np.int64), np.zeros(n, np.int64), np.zeros(n, np.int64)
+        self._check(lib().ccsim_debug_node_scores(self._h, t, clones, total.ctypes.data_as(abi.P64), least.ctypes.data_as(abi.P64),
+                                                  balanced.ctypes.data_as(abi.P64)), "ccsim_debug_node_scores")
+        return total[: self._n], least[: self._n], balanced[: self._n]
 
     def kernel_launches(self):
         return int(lib().ccsim_kernel_launches(self._h))

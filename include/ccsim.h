@@ -317,11 +317,25 @@ int  ccsim_peer_import_local(ccsim_handle *h, int32_t world, void *const *ptrs /
 int  ccsim_device_info(ccsim_handle *h, int32_t *sm_count, int32_t *grid, int32_t *block, int64_t *l2_bytes);
 int64_t ccsim_kernel_launches(const ccsim_handle *h);  /* kernels launched by this handle so far */
 int  ccsim_flush_l2(ccsim_handle *h);                  /* writes a buffer larger than L2 (bench hygiene) */
-/* latency anatomy of the last run (bench.py's roofline block): [0] engine (0 generic, 1 lean sequential, 2 tie-run batching,
- * 3 multi-commit, 4 streaming) [1] waves [2] placed [3] multi-commit: candidates replayed, summed over waves [4] multi-commit: waves that
- * raised the candidate bar [5] grid [6] block [7] dynamic shared memory bytes [8..15] CTA 0's clock cycles per phase, summed
- * over waves (multi-commit: scan, barrier, merge+publish, gather, replay, row updates+recount; 0 for the other engines) */
+/* latency anatomy of the last run (bench.py's roofline block): [0] engine in the low byte (0 generic, 1 lean sequential, 2 tie-run
+ * batching, 3 multi-commit, 4 streaming), CCSIM_KV_* bits above it [1] waves [2] placed [3] multi-commit: candidates replayed, summed
+ * over waves [4] multi-commit: waves that raised the candidate bar [5] grid [6] block [7] multi-commit: replay rounds, summed over
+ * waves [8..15] CTA 0's clock cycles per phase, summed over waves (multi-commit: scan, barrier, merge+publish, gather, replay, row
+ * updates+recount; 0 for the other engines) */
 int  ccsim_run_stats(const ccsim_handle *h, int64_t out[16]);
+/* which instantiation of the engine's wave kernel ran (ccsim_run_stats out[0]) */
+#define CCSIM_KV_ENGINE_MASK          0xffll
+#define CCSIM_KV_RESIDENT             (1ll << 8)   /* generic kernel: the node tile stays in shared memory (else columns are re-read from L2) */
+#define CCSIM_KV_STREAM_MODE_SHIFT    9            /* streaming kernel: 2 bits, MODE 0 (every column streamed), 1 (+ taint/static words),
+                                                      2 (free columns resident, only the score memo streamed) */
+#define CCSIM_KV_REFERENCE_SAMPLING   (1ll << 11)  /* lean kernel in CCSIM_SAMPLING_REFERENCE mode */
+#define CCSIM_KV_CROSS_GPU            (1ll << 12)  /* multi-commit kernel of a node-sharded run (world > 1) */
+
+/* Scores node i of the loaded snapshot (this handle's shard, [n] entries each) for template t as if `clones` pods of t had been
+ * committed to it, with the device function every wave kernel scores with: total = NodeResourcesFit (LeastAllocated) * w_fit +
+ * BalancedAllocation * w_balanced as enabled by the template, least / balanced = the unweighted plugin scores. The other plugins'
+ * shares (TaintToleration, NodeAffinity, ...) are not part of it. Needs ccsim_set_templates; does not touch the run state. */
+int  ccsim_debug_node_scores(ccsim_handle *h, int32_t t, int32_t clones, int64_t *total, int64_t *least, int64_t *balanced);
 
 #ifdef __cplusplus
 }

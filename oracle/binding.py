@@ -80,3 +80,15 @@ def node_score(snapshot, template, i, clones):
     l, b = C.c_int64(), C.c_int64()
     tot = lib().ccsim_oracle_node_score(C.byref(nd), C.byref(template), i, clones, C.byref(l), C.byref(b))
     return int(tot), int(l.value), int(b.value)
+
+
+def node_scores(snapshot, template, clones):
+    """node_score of every node: (total, least, balanced) int64 arrays."""
+    nd = snapshot.c_struct()
+    f = lib().ccsim_oracle_node_score
+    l, b = C.c_int64(), C.c_int64()
+    out = np.zeros((3, snapshot.n), np.int64)
+    for i in range(snapshot.n):
+        out[0, i] = f(C.byref(nd), C.byref(template), i, clones, C.byref(l), C.byref(b))
+        out[1, i], out[2, i] = l.value, b.value
+    return out[0], out[1], out[2]
